@@ -285,11 +285,45 @@ def gen_losses():
     save("losses", dict(kind="losses"), **arrays)
 
 
+def gen_checkpoint():
+    """The training checkpoint the reference writes (bin/train.py:112-146): a HiFi-GAN generator after one RAdam step
+    on seeded gradients, the default multi-scale multi-period discriminator and a fresh Adam for it.  Stored: the
+    layouts (state-dict names + shapes, optimizer groups, optimizer state keys), the seeds, checksums of every tensor
+    group and the first parameter's optimizer state.  The tensors themselves are rebuilt from the seeds by the test."""
+    import parallel_wavegan.models as M
+    from parallel_wavegan.optimizers import RAdam
+
+    kwargs = dict(in_channels=80, out_channels=1, channels=64, kernel_size=7, upsample_scales=[8, 8, 2, 2],
+                  upsample_kernel_sizes=[16, 16, 4, 4], resblock_kernel_sizes=[3, 7, 11],
+                  resblock_dilations=[[1, 3, 5], [1, 3, 5], [1, 3, 5]])
+    torch.manual_seed(0)
+    g, d = M.HiFiGANGenerator(**kwargs), M.HiFiGANMultiScaleMultiPeriodDiscriminator()
+    g_spec, _ = load_synth(g, 11, 1.0)
+    d_spec, _ = load_synth(d, 12, 1.0)
+    opt_g = RAdam(g.parameters(), lr=1e-3)
+    for i, p in enumerate(g.parameters()):
+        p.grad = synth.randn(p.shape, 5000 + i, 0.01)
+    opt_g.step()
+    sd_g, sd_d = opt_g.state_dict(), torch.optim.Adam(d.parameters()).state_dict()
+    state = [sd_g["state"][i] for i in range(len(sd_g["state"]))]
+    meta = dict(kind="checkpoint", g_kwargs=kwargs, g_spec=g_spec, g_seed=11, d_spec=d_spec, d_seed=12, gain=1.0,
+                grad_seed=5000, grad_scale=0.01, g_param_groups=sd_g["param_groups"], d_param_groups=sd_d["param_groups"],
+                state_keys=list(state[0].keys()), step=state[0]["step"],
+                g_checksum=synth.checksum(g.state_dict()), d_checksum=synth.checksum(d.state_dict()),
+                exp_avg_checksum=synth.checksum({i: s["exp_avg"] for i, s in enumerate(state)}),
+                exp_avg_sq_checksum=synth.checksum({i: s["exp_avg_sq"] for i, s in enumerate(state)}))
+    save("checkpoint_ref", meta, exp_avg_p0=state[0]["exp_avg"], exp_avg_sq_p0=state[0]["exp_avg_sq"])
+
+
 def main():
     import_reference()
     if "style_disc" in sys.argv[1:]:  # regenerate only the fixture added in round 2
         gen_discriminator("style_melgan_disc", "StyleMelGANDiscriminator", {}, B=2, T=6000, seed=65, gain=1.4, np_seed=21, keep=("_filter",))
         return
+    if "checkpoint" in sys.argv[1:]:  # regenerate only the checkpoint-interchange fixture
+        gen_checkpoint()
+        return
+    gen_checkpoint()
     gen_losses()
     gen_discriminator("style_melgan_disc", "StyleMelGANDiscriminator", {}, B=2, T=6000, seed=65, gain=1.4, np_seed=21, keep=("_filter",))
     gen_discriminator("hifigan_msmpd_v1", "HiFiGANMultiScaleMultiPeriodDiscriminator", {}, B=2, T=8192, seed=61, gain=1.4)

@@ -1,15 +1,14 @@
 """Checkpoint boundary (CPU, no kernels): ``utils.load_model`` (utils/utils.py:294-360) and the
-``Trainer.save_checkpoint`` dict layout (bin/train.py:112-186) round-trip through the mirror modules; when the
-reference tree is present (build container) checkpoints written by the REAL reference load into the mirror and
-checkpoints written by the mirror load strictly into the reference modules."""
-import os
+``Trainer.save_checkpoint`` dict layout (bin/train.py:112-186) round-trip through the mirror modules; a checkpoint
+written by the REAL reference (rebuilt from tests/golden/checkpoint_ref.npz) loads into the mirror and checkpoints
+written by the mirror have the layout the reference modules and optimizer load."""
 import sys
 
 import numpy as np
-import pytest
 import torch
 import yaml
 
+from helpers import load_golden
 from oracle import synth
 
 HIFI_SMALL = dict(in_channels=80, out_channels=1, channels=64, kernel_size=7, upsample_scales=[8, 8, 2, 2],
@@ -91,44 +90,65 @@ def test_load_model_from_checkpoint_dir(tmp_path):
     assert isinstance(mh, models.HiFiGANGenerator)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/parallel_wavegan"), reason="reference tree only exists in the build container")
+def _reference_checkpoint(meta, gold):
+    """The checkpoint the real reference wrote (tests/golden/checkpoint_ref.npz, oracle/make_golden.py), rebuilt from
+    its seeds: synthetic weights, one RAdam step (oracle.ref_optim.radam_step, the reference's own tensor ops) on
+    seeded gradients; checked against the checksums and the first parameter's state the reference recorded."""
+    from oracle import ref_optim
+
+    g_sd = synth.synth_state_dict(meta["g_spec"], meta["g_seed"], meta["gain"])
+    d_sd = synth.synth_state_dict(meta["d_spec"], meta["d_seed"], meta["gain"])
+    (group,) = meta["g_param_groups"]
+    assert len(group["params"]) == len(g_sd)  # every generator state-dict entry is a parameter, in parameter order
+    state = {}
+    for i, p in enumerate(g_sd.values()):
+        m, v = torch.zeros_like(p), torch.zeros_like(p)
+        grad = synth.randn(p.shape, meta["grad_seed"] + i, meta["grad_scale"])
+        ref_optim.radam_step(p, grad, m, v, meta["step"], group["lr"], tuple(group["betas"]), group["eps"], group["weight_decay"])
+        s = {"step": meta["step"], "exp_avg": m, "exp_avg_sq": v}
+        state[i] = {k: s[k] for k in meta["state_keys"]}
+    for sd, key in ((g_sd, "g_checksum"), (d_sd, "d_checksum"),
+                    ({i: s["exp_avg"] for i, s in state.items()}, "exp_avg_checksum"),
+                    ({i: s["exp_avg_sq"] for i, s in state.items()}, "exp_avg_sq_checksum")):
+        assert abs(synth.checksum(sd) - meta[key]) <= 1e-12 * abs(meta[key]), key
+    assert torch.equal(state[0]["exp_avg"], gold["exp_avg_p0"]) and torch.equal(state[0]["exp_avg_sq"], gold["exp_avg_sq_p0"])
+    groups = {net: [dict(gr, betas=tuple(gr["betas"])) for gr in meta[f"{net[0]}_param_groups"]] for net in ("generator", "discriminator")}
+    return {"model": {"generator": g_sd, "discriminator": d_sd},
+            "optimizer": {"generator": {"state": state, "param_groups": groups["generator"]},
+                          "discriminator": {"state": {}, "param_groups": groups["discriminator"]}},
+            "scheduler": {"generator": {}, "discriminator": {}}, "steps": 1, "epochs": 0}
+
+
 def test_checkpoints_interchange_with_the_real_reference(tmp_path):
-    from oracle.make_golden import import_reference
-
-    import_reference()
-    import parallel_wavegan.models as rm
-    from parallel_wavegan.optimizers import RAdam as RefRAdam
-
     from parallelwavegan_b200 import models, optimizers, utils
 
+    meta, gold = load_golden("checkpoint_ref")
+    assert meta["g_kwargs"] == HIFI_SMALL
+
     # reference -> mirror
-    rg, rd = rm.HiFiGANGenerator(**HIFI_SMALL), rm.HiFiGANMultiScaleMultiPeriodDiscriminator()
-    _fill(rg, 11)
-    _fill(rd, 12)
-    ro = RefRAdam(rg.parameters(), lr=1e-3)
-    for p in rg.parameters():
-        p.grad = torch.randn_like(p) * 0.01
-    ro.step()
+    ck_ref = _reference_checkpoint(meta, gold)
     path = str(tmp_path / "ref.pkl")
-    torch.save({"model": {"generator": rg.state_dict(), "discriminator": rd.state_dict()},
-                "optimizer": {"generator": ro.state_dict(), "discriminator": torch.optim.Adam(rd.parameters()).state_dict()},
-                "scheduler": {"generator": {}, "discriminator": {}}, "steps": 1, "epochs": 0}, path)
+    torch.save(ck_ref, path)
     m = utils.load_model(path, config={"generator_type": "HiFiGANGenerator", "generator_params": HIFI_SMALL, "format": "npy"})
-    for (k, a), (k2, b) in zip(rg.state_dict().items(), m.state_dict().items()):
+    for (k, a), (k2, b) in zip(ck_ref["model"]["generator"].items(), m.state_dict().items()):
         assert k == k2 and torch.equal(a, b)
     g2, d2 = models.HiFiGANGenerator(**HIFI_SMALL), models.HiFiGANMultiScaleMultiPeriodDiscriminator()
     o2 = optimizers.RAdam(g2.parameters(), lr=1.0)
     utils.load_checkpoint(path, {"generator": g2, "discriminator": d2}, {"generator": o2, "discriminator": optimizers.FusedAdam(d2.parameters())})
-    p_ref, p_new = next(iter(rg.parameters())), next(iter(g2.parameters()))
-    assert torch.equal(ro.state[p_ref]["exp_avg"], o2.state[p_new]["exp_avg"]) and o2.state[p_new]["step"] == 1
+    p_new = next(iter(g2.parameters()))
+    assert torch.equal(gold["exp_avg_p0"], o2.state[p_new]["exp_avg"]) and o2.state[p_new]["step"] == 1
     assert o2.param_groups[0]["lr"] == 1e-3
-    # mirror -> reference (strict)
+    # mirror -> reference: a strict load_state_dict into the reference modules needs the same names and shapes
     utils.save_checkpoint(str(tmp_path / "ours.pkl"), {"generator": g2, "discriminator": d2},
                           {"generator": o2, "discriminator": optimizers.FusedAdam(d2.parameters())})
     ck = torch.load(str(tmp_path / "ours.pkl"), map_location="cpu")
-    rg2, rd2 = rm.HiFiGANGenerator(**HIFI_SMALL), rm.HiFiGANMultiScaleMultiPeriodDiscriminator()
-    rg2.load_state_dict(ck["model"]["generator"], strict=True)
-    rd2.load_state_dict(ck["model"]["discriminator"], strict=True)
-    ro2 = RefRAdam(rg2.parameters(), lr=5.0)
+    for net in ("generator", "discriminator"):
+        assert {k: list(v.shape) for k, v in ck["model"][net].items()} == {k: s for k, s in meta[f"{net[0]}_spec"]}, net
+    # the reference RAdam inherits load_state_dict from torch.optim.Optimizer (radam.py) and its step() reads the
+    # state keys it writes
+    (group,) = meta["g_param_groups"]
+    ro2 = torch.optim.Optimizer([torch.nn.Parameter(torch.zeros(s)) for _, s in meta["g_spec"]],
+                                dict({k: v for k, v in group.items() if k != "params"}, lr=5.0))
     ro2.load_state_dict(ck["optimizer"]["generator"])
     assert ro2.param_groups[0]["lr"] == 1e-3
+    assert all(sorted(s) == sorted(meta["state_keys"]) for s in ck["optimizer"]["generator"]["state"].values())
